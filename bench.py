@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the FastMOT per-frame hot path on B200 (BASELINE.json metric: frames/sec/stream @1080p, 200 tracks).
 
-    python bench.py --gpus N --steps K --warmup W [--config 3] [--repeats R]   # our arm (one process per GPU)
+    python bench.py --gpus N --steps K --warmup W [--config 3] [--repeats R] [--dump-outputs DIR]   # our arm
     python bench.py --impl reference --steps K --warmup W [--config 3]         # reference CPU arm (host cores)
 
 A "step" is one `MOT.step(frame)` on the next 1920x1080 frame of a deterministic synthetic stream.  `--config`
@@ -15,14 +15,21 @@ ground-truth boxes AFTER the whole detector pipeline (letterbox, conv stack, dec
 random weights cannot detect, and the tracker must see the tracks.  Everything else is real data flow: ReID crops come
 from the frame, OSNet embeddings feed the association kernels.
 
-Timing: W warm-up steps (the conv engines are additionally replayed 3 times at build), then R windows of exactly K
-steps, each bracketed by barrier + synchronize, CUDA events on the launching stream, max over ranks; the line reports
-the MEDIAN window (`repeats` holds min / max).
-`value`  : frames already resident in HBM (all distinct, > L2 in total) when the timed region starts.
+Timing: W warm-up steps (at least two detector periods after init; the conv engines are additionally replayed 3 times
+at build), then R windows of exactly K steps (R = 1 by default, so K steps are timed), each bracketed by barrier +
+synchronize, CUDA events on the launching stream, max over ranks; the line reports the MEDIAN window (`repeats` holds
+min / max).
+`value`  : frames already resident in HBM (all distinct; their total size is in `config.l2`) when the timed region
+           starts.
 `e2e`    : the same steps through the public API with frames in pinned HOST memory (6.2 MB H2D inside every step,
            track ids / boxes read back every step; bytes counted from the arrays actually copied).
 `roofline_stages`: a third pass with per-stage CUDA events (fastmot_b200/stagetime.py) -> ms per call, algorithmic
            bytes / flops (SURVEY.md 8d figures), fraction of the measured peak or "latency" for the serial stages.
+
+--dump-outputs DIR writes what the caller holds after the last timed step of the `value` pass (rank 0's stream): the
+visible tracks' ids, boxes, labels, Kalman mean / covariance and running-mean ReID embedding, one DIR/<name>.npy each.
+The stream, the scripted detections and the synthetic weights are seeded, so two builds run with the same arguments
+can be compared array by array.
 """
 import argparse
 import json
@@ -114,6 +121,29 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def track_outputs(tracks, feat_dim):
+    """What a caller of MOT.step / MultiTracker reads from the visible tracks, as float32 / float64 arrays."""
+    tracks = list(tracks)
+    n = len(tracks)
+    states = [t.state for t in tracks]
+    feats = [t.avg_feat() for t in tracks]
+    return {
+        "track_ids": np.array([t.trk_id for t in tracks], np.float64),
+        "track_tlbr": np.array([t.tlbr for t in tracks], np.float64).reshape(n, 4),
+        "track_label": np.array([t.label for t in tracks], np.float64),
+        "track_mean": np.array([m for m, _ in states], np.float64).reshape(n, 8),
+        "track_cov": np.array([c for _, c in states], np.float64).reshape(n, 8, 8),
+        "track_feature": np.array([np.zeros(feat_dim, np.float32) if f is None else f for f in feats],
+                                  np.float32).reshape(n, feat_dim),
+    }
+
+
+def dump_outputs(arrays, out_dir):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def make_scene(c, seed):
@@ -242,7 +272,11 @@ def run_ours(args):
     from fastmot_b200 import engine as eng_mod
     _lib.require_device()
     c = CONFIGS[args.config]
-    K, W, R = args.steps, args.warmup, args.repeats
+    # the first detector periods after init are transient (the association update at frame `skip` is the first one and
+    # the tracks have no history yet): the warm-up always covers two periods, so the timed window is steady state
+    K, W, R = args.steps, max(args.warmup, 2 * c["skip"]), args.repeats
+    sampler = ClockSampler(local)
+    sampler.start()          # nvidia-smi needs ~1 s to start and slows launches meanwhile: start before the model build
     dev = torch.device("cuda", local)
     scene = make_scene(c, rank)
     total = W + R * K
@@ -286,8 +320,9 @@ def run_ours(args):
             mot.step(f)
             return sum(1 for _ in mot.visible_tracks())
 
-        def readback_bytes():
-            return sum(t.tlbr.nbytes + 8 for t in mot.visible_tracks())
+        def visible():
+            return mot.visible_tracks()
+        tracker = mot.tracker
     else:
         from fastmot_b200 import MultiTracker
         from fastmot_b200.config import default_tracker_cfg
@@ -314,20 +349,24 @@ def run_ours(args):
             state["t"] = t + 1
             return sum(1 for v in trk.tracks.values() if v.confirmed and v.active)
 
-        def readback_bytes():
-            return sum(v.tlbr.nbytes + 8 for v in trk.tracks.values() if v.confirmed and v.active)
+        def visible():
+            return (v for v in trk.tracks.values() if v.confirmed and v.active)
+        tracker = trk
+
+    def readback_bytes():
+        return sum(t.tlbr.nbytes + 8 for t in visible())
 
     prof = eng_mod.enable_profiling()
-    sampler = ClockSampler(local)
-    sampler.start()          # nvidia-smi needs ~1 s before its first sample: start before the warm-up
 
     def run_pass(inputs, prefetch=False):
         """W warm-up steps, then R windows of K steps.  Returns per-window ms (max over ranks), per-step ms of the last
         window, visible tracks.  prefetch: MOT.prefetch(next frame) before every step (read-ahead upload stream)."""
         reset()
-        for f in inputs[:W]:
-            step(f)
         pre = (lambda f: mot.prefetch(f)) if (prefetch and c["kind"] == "mot") else None
+        for i, f in enumerate(inputs[:W]):
+            if pre is not None:          # the first timed frame arrives prefetched, like every later one
+                pre(inputs[i + 1])
+            step(f)
         win_ms, step_ms, n_vis = [], [], 0
         for r in range(R):
             chunk = inputs[W + r * K: W + (r + 1) * K]
@@ -351,8 +390,9 @@ def run_ours(args):
     launches0 = _lib.launch_count()
     win_dev, step_dev, n_vis = run_pass(dev_frames)
     launches = (_lib.launch_count() - launches0)
-    clocks = sampler.stop()
     conv = prof.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(track_outputs(visible(), tracker.pool.feat_dim), args.dump_outputs)
     # ---- pass 2: end to end from pinned host memory through the public API ----
     if c["kind"] == "mot":
         host_frames = [torch.as_tensor(f).pin_memory().numpy() for f in frames]
@@ -360,6 +400,7 @@ def run_ours(args):
     else:
         host_frames, h2d = frames, int(scene.detections(0)[0].nbytes + 64 * 512 * 4)
     win_e2e, _, _ = run_pass(host_frames, prefetch=not args.no_prefetch)
+    clocks = sampler.stop()          # over both timed passes: one window of K steps can be shorter than a sample
     d2h = int(readback_bytes())
     # ---- pass 3: per-stage CUDA events (not part of the timed numbers above) ----
     prof.reset()
@@ -392,7 +433,8 @@ def run_ours(args):
             "config": {"workload": c["workload"], "config_id": args.config, "streams": world,
                        "value_is": "aggregate over all streams (one stream per GPU); per-stream = value / n_gpus",
                        "parallelism": f"{world} independent streams, one per GPU, no collective",
-                       "l2": f"{W + R * K} distinct frames (6.2 MB each, > 126 MB L2 in total) -- inputs larger than L2",
+                       "l2": (f"{W + R * K} distinct frames, 6.2 MB each: {(W + R * K) * 6.22:.0f} MB in total "
+                              "(B200 L2: 126 MB)") if c["kind"] == "mot" else "no frames",
                        "detections": "scripted ground-truth boxes replace the detector output rows after the full "
                                      "detector pipeline ran (random weights cannot detect)",
                        "visible_tracks_last_step": int(n_vis), "conv_path": conv.get("conv_path"),
@@ -537,7 +579,7 @@ if __name__ == "__main__":
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=40)
     ap.add_argument("--warmup", type=int, default=10)
-    ap.add_argument("--repeats", type=int, default=5)
+    ap.add_argument("--repeats", type=int, default=1, help="timed windows of --steps steps each")
     ap.add_argument("--config", type=int, default=3, choices=sorted(CONFIGS))
     ap.add_argument("--p5-input", type=int, default=896, choices=[896, 1280])
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -545,6 +587,8 @@ if __name__ == "__main__":
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-nets", action="store_true")
     ap.add_argument("--no-prefetch", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the visible tracks after the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
     if a.impl == "reference":
         run_reference(a)

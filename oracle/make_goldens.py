@@ -166,9 +166,75 @@ def primitive_golden():
     print('assoc_primitives', k)
 
 
+# scenes of tests/test_oracle_vs_reference.py (same order, same frame counts)
+PARITY_SCENES = [
+    (dict(n_objects=40, seed=9), 17),
+    (dict(n_objects=30, seed=4, overlap=True), 12),
+    (dict(n_objects=64, seed=1), 22),
+    (dict(n_objects=50, seed=7, bounce_radius=8), 31),
+    (dict(n_objects=30, seed=12, dropout_frames=(10,), dropout_every=1), 22),
+    (dict(n_objects=30, seed=13, dropout_frames=(5, 10, 15), dropout_every=2), 22),
+]
+
+# det.txt of tests/test_public_detector.py
+PUBLIC_DET_TXT = """1,-1,100.4,200.6,50.5,120.2,0.9,-1,-1,-1
+1,-1,1800.0,900.0,200.0,300.0,0.4,-1,-1,-1
+2,-1,10,20,30,40,1,-1,-1,-1
+6,-1,640.5,360.5,11,21,1,-1,-1,-1
+6,-1,0,0,1919,1079,1,-1,-1,-1
+"""
+PUBLIC_SIZES = ((1280, 720), (1920, 1080), (640, 360))
+
+
+def parity_golden():
+    """What the reference itself outputs for the oracle-parity tests: the full tracker (MultiTracker + Flow) on the
+    PARITY_SCENES, DIoU-NMS on random boxes and the MOT Challenge public-detection reader."""
+    import tempfile
+    fm = load_reference()
+    rec = {'n_scenes': np.int64(len(PARITY_SCENES))}
+    for i, (scene_kw, n_frames) in enumerate(PARITY_SCENES):
+        out, trk = run_reference_tracker(SyntheticScene(**scene_kw), n_frames)
+        rec[f's{i}_scene_kw'] = np.array(repr(scene_kw))
+        rec[f's{i}_n_frames'] = np.int64(n_frames)
+        for t, o in enumerate(out):
+            rec[f's{i}_ids_{t}'] = o['ids']
+            rec[f's{i}_tlbr_{t}'] = o['tlbr']
+        keys = np.array(list(trk.tracks.keys()), np.int64)
+        rec[f's{i}_track_ids'] = keys
+        rec[f's{i}_homography'] = np.array(trk.homography, np.float64)
+        rec[f's{i}_mean'] = np.array([trk.tracks[k].state[0] for k in keys], np.float64).reshape(-1, 8)
+    rng = np.random.default_rng(3)
+    rec['n_nms'] = np.int64(6)
+    for k in range(6):
+        n = int(rng.integers(5, 150))
+        tlwh = np.concatenate([rng.uniform(0, 300, (n, 2)), rng.uniform(10, 120, (n, 2))], 1).astype(np.float32)
+        sc = rng.uniform(0.3, 1, n).astype(np.float32)
+        rec[f'nms_tlwh_{k}'], rec[f'nms_score_{k}'] = tlwh, sc
+        rec[f'nms_keep_{k}'] = np.array(fm.utils.rect.diou_nms(tlwh, sc, 0.5), np.int64)
+    rec['pub_det_txt'] = np.array(PUBLIC_DET_TXT)
+    with tempfile.TemporaryDirectory() as tmp:
+        seq = os.path.join(tmp, 'MOT-TEST')
+        os.makedirs(os.path.join(seq, 'det'))
+        with open(os.path.join(seq, 'seqinfo.ini'), 'w') as f:
+            f.write("[Sequence]\nname=MOT-TEST\nimWidth=1920\nimHeight=1080\n")
+        with open(os.path.join(seq, 'det', 'det.txt'), 'w') as f:
+            f.write(PUBLIC_DET_TXT)
+        for j, size in enumerate(PUBLIC_SIZES):
+            det = fm.detector.PublicDetector(size, (1,), 5, sequence_path=seq, conf_thresh=0.5, max_area=800000)
+            for c in range(3):
+                d = det.postprocess()
+                rec[f'pub_tlbr_{j}_{c}'] = np.array(d.tlbr, np.float64).reshape(-1, 4)
+                rec[f'pub_label_{j}_{c}'] = np.array(d.label, np.int64)
+                rec[f'pub_conf_{j}_{c}'] = np.array(d.conf, np.float64)
+    np.savez_compressed(os.path.join(OUT, 'reference_parity.npz'), **rec)
+    print('reference_parity', len(PARITY_SCENES), 'scenes')
+
+
 if __name__ == '__main__':
     os.makedirs(OUT, exist_ok=True)
-    which = sys.argv[1:] or ['prim', 'seq64', 'seq200', 'seqovl']
+    which = sys.argv[1:] or ['prim', 'seq64', 'seq200', 'seqovl', 'parity']
+    if 'parity' in which:
+        parity_golden()
     if 'prim' in which:
         primitive_golden()
     if 'seq64' in which:

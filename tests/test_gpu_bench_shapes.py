@@ -76,3 +76,39 @@ def test_config2_detector_every_frame_tiny_x025():
     frac, n = _run('YOLOv4Tiny', 'OSNet025', 50, 1, 8, seed=5)
     assert n == 50
     assert frac > 0.7, frac
+
+
+def test_bench_dump_outputs_repeatable_and_taken_after_the_last_timed_step(tmp_path):
+    """`bench.py --dump-outputs`: the same arguments give the same arrays (float32 / float64, within the 64 MB
+    budget); one more timed step moves the tracks."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from conftest import ROOT
+    names = {"track_ids", "track_tlbr", "track_label", "track_mean", "track_cov", "track_feature"}
+
+    def run(steps, tag):
+        out = tmp_path / tag
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--config", "1", "--steps", str(steps),
+                            "--warmup", "2", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == steps and line["repeats"]["windows"] == 1
+        assert {p.stem for p in out.iterdir()} == names
+        arrays = {n: np.load(out / f"{n}.npy") for n in names}
+        assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+        assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+        return arrays, line
+
+    a, line = run(3, "a")
+    n = len(a["track_ids"])
+    assert n == line["config"]["visible_tracks_last_step"] > 0
+    assert a["track_tlbr"].shape == (n, 4) and a["track_cov"].shape == (n, 8, 8)
+    assert a["track_feature"].shape == (n, 512)
+    b, _ = run(3, "b")
+    for k in names:
+        np.testing.assert_array_equal(a[k], b[k], err_msg=k)
+    c, _ = run(4, "c")
+    assert not np.array_equal(a["track_mean"], c["track_mean"])

@@ -1,11 +1,23 @@
-"""CPU, build container only: the oracle restatements against the UNMODIFIED reference imported from
-/root/reference (skipped where the reference tree is absent, e.g. on the GPU box)."""
+"""CPU: the oracle restatements against what the UNMODIFIED reference outputs on the same inputs, stored in
+tests/golden/reference_parity.npz (written from the reference by `python -m oracle.make_goldens parity`)."""
+import os
+
 import numpy as np
 import pytest
 
-from oracle.refshim import reference_available
+from conftest import GOLDEN
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree not present")
+
+@pytest.fixture(scope="module")
+def parity():
+    return np.load(os.path.join(GOLDEN, "reference_parity.npz"))
+
+
+def _scene_index(g, scene_kw, n_frames):
+    for i in range(int(g['n_scenes'])):
+        if str(g[f's{i}_scene_kw']) == repr(scene_kw) and int(g[f's{i}_n_frames']) == n_frames:
+            return i
+    raise KeyError(f"no reference golden for {scene_kw!r}, {n_frames} frames")
 
 
 @pytest.mark.parametrize("scene_kw,n_frames", [
@@ -17,30 +29,25 @@ pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tre
     (dict(n_objects=30, seed=12, dropout_frames=(10,), dropout_every=1), 22),       # a detector frame with NO detections
     (dict(n_objects=30, seed=13, dropout_frames=(5, 10, 15), dropout_every=2), 22),  # half the objects never confirm
 ])
-def test_oracle_tracker_full_pipeline_identical(scene_kw, n_frames):
+def test_oracle_tracker_full_pipeline_identical(parity, scene_kw, n_frames):
     """OracleTracker + OracleFlow (cv2) vs reference MultiTracker + Flow: identical ids and boxes per frame."""
     from fastmot_b200.synth import SyntheticScene
-    from oracle.ref_run import run_reference_tracker
     from oracle.run import run_oracle_tracker
-    scene = SyntheticScene(**scene_kw)
-    ref, rtrk = run_reference_tracker(scene, n_frames)
+    i = _scene_index(parity, scene_kw, n_frames)
     got, otrk = run_oracle_tracker(SyntheticScene(**scene_kw), n_frames)
     for t in range(n_frames):
-        assert np.array_equal(ref[t]['ids'], got[t]['ids']), t
-        assert np.array_equal(ref[t]['tlbr'], got[t]['tlbr']), t
-    assert list(rtrk.tracks.keys()) == list(otrk.tracks.keys())
-    np.testing.assert_allclose(rtrk.homography, otrk.homography, atol=1e-12)
-    for k in rtrk.tracks:
-        np.testing.assert_allclose(rtrk.tracks[k].state[0], otrk.tracks[k].mean, atol=1e-6)
+        assert np.array_equal(parity[f's{i}_ids_{t}'], got[t]['ids']), t
+        assert np.array_equal(parity[f's{i}_tlbr_{t}'], got[t]['tlbr']), t
+    ref_ids = parity[f's{i}_track_ids']
+    assert ref_ids.tolist() == list(otrk.tracks.keys())
+    np.testing.assert_allclose(parity[f's{i}_homography'], otrk.homography, atol=1e-12)
+    for k, mean in zip(ref_ids.tolist(), parity[f's{i}_mean']):
+        np.testing.assert_allclose(mean, otrk.tracks[k].mean, atol=1e-6)
 
 
-def test_detect_oracle_against_reference_functions():
-    from oracle.refshim import load_reference
+def test_detect_oracle_against_reference_functions(parity):
     from oracle import detect
-    fm = load_reference()
-    rng = np.random.default_rng(3)
+    assert int(parity['n_nms']) == 6
     for trial in range(6):
-        n = int(rng.integers(5, 150))
-        tlwh = np.concatenate([rng.uniform(0, 300, (n, 2)), rng.uniform(10, 120, (n, 2))], 1).astype(np.float32)
-        sc = rng.uniform(0.3, 1, n).astype(np.float32)
-        assert np.array_equal(fm.utils.rect.diou_nms(tlwh, sc, 0.5), detect.diou_nms(tlwh, sc, 0.5))
+        tlwh, sc = parity[f'nms_tlwh_{trial}'], parity[f'nms_score_{trial}']
+        assert np.array_equal(parity[f'nms_keep_{trial}'], detect.diou_nms(tlwh, sc, 0.5))

@@ -1,11 +1,10 @@
 """SURVEY.md §8(f) row 2: MOT Challenge public-detection reader and result writer (host-side formats either side of
-the hot path).  The reader is checked against hand-computed rows and, in the build container, against the
-reference's own `PublicDetector` imported through oracle/refshim.py."""
+the hot path).  The reader is checked against hand-computed rows and against the rows the reference's own
+`PublicDetector` returned for the same det.txt (tests/golden/reference_parity.npz)."""
 import io
 import os
 
 import numpy as np
-import pytest
 
 DET_TXT = """1,-1,100.4,200.6,50.5,120.2,0.9,-1,-1,-1
 1,-1,1800.0,900.0,200.0,300.0,0.4,-1,-1,-1
@@ -44,21 +43,19 @@ def test_public_detector_rows(tmp_path):
     np.testing.assert_array_equal(d5b.tlbr[1], [0, 0, 1279, 719])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/fastmot"), reason="reference tree only in the build container")
-def test_public_detector_matches_reference(tmp_path):
-    from oracle import refshim
-    ref = refshim.load_reference()
+def test_public_detector_matches_reference(tmp_path, golden_dir):
     from fastmot_b200 import PublicDetector
+    g = np.load(os.path.join(golden_dir, "reference_parity.npz"))
+    assert str(g["pub_det_txt"]) == DET_TXT
     seq = _make_sequence(tmp_path, 1920, 1080)
-    for size in ((1280, 720), (1920, 1080), (640, 360)):
+    for j, size in enumerate(((1280, 720), (1920, 1080), (640, 360))):
         ours = PublicDetector(size, (1,), 5, sequence_path=str(seq), conf_thresh=0.5, max_area=800000)
-        theirs = ref.detector.PublicDetector(size, (1,), 5, sequence_path=str(seq), conf_thresh=0.5, max_area=800000)
-        for _ in range(3):
-            a, b = ours.postprocess(), theirs.postprocess()
-            assert len(a) == len(b)
-            np.testing.assert_array_equal(a.tlbr, b.tlbr)
-            np.testing.assert_array_equal(a.label, b.label)
-            np.testing.assert_array_equal(a.conf, b.conf)
+        for c in range(3):
+            a = ours.postprocess()
+            assert len(a) == len(g[f"pub_tlbr_{j}_{c}"])
+            np.testing.assert_array_equal(a.tlbr, g[f"pub_tlbr_{j}_{c}"])
+            np.testing.assert_array_equal(a.label, g[f"pub_label_{j}_{c}"])
+            np.testing.assert_array_equal(a.conf, g[f"pub_conf_{j}_{c}"])
 
 
 def test_mot_result_line_format():
